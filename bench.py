@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (one rank per GPU under torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU dmrecon on the host cores
     python bench.py --workload C3|C4|C5 --gpus N ...         # the other BASELINE configs (nominally 8 / 4 / 8 GPUs)
+    python bench.py ... --dump-outputs DIR                   # also write the maps of the last timed step (dump_outputs)
 
 Workload (default, N = 1): BASELINE.json configs[1] (C2) - synthetic 16-view 1920x1080 scene, dmrecon scale = 1, all 16
 views reconstructed; one step = DMRecon::start for all 16 reference views.  N > 1: the same per-GPU work (16 reference
@@ -226,6 +227,25 @@ def reference_arm(args, real_stdout):
 # ----------------------------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 << 20          # what --dump-outputs writes in all, headers aside
+
+
+def dump_outputs(path, bufs):
+    """Writes the maps a caller of the timed step receives, one row per reference view in order: depth.npy [V, P],
+    conf.npy [V, P] and dz.npy [V, P, 2], float32.  P is every pixel of the map, row-major, or, when that would exceed
+    DUMP_BYTES, the same sample of pixels in every view: np.sort(np.random.default_rng(0).choice(H * W, P, replace=False)).
+    The frontier schedule is not bitwise reproducible at this size, so compare with a tolerance: two runs of the same build
+    on C2 (one B200, 1000 W power limit) differed in 0.2-0.7 % of these values, depth by at most 8e-4 relative, with
+    identical fill masks."""
+    h, w = bufs[0]["depth"].shape
+    n = min(h * w, DUMP_BYTES // (16 * len(bufs)))
+    idx = np.arange(h * w) if n == h * w else np.sort(np.random.default_rng(0).choice(h * w, n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for k, shape in (("depth", (-1,)), ("conf", (-1,)), ("dz", (-1, 2))):
+        np.save(os.path.join(path, k + ".npy"), np.stack([b[k].reshape(shape)[idx] for b in bufs]).astype(np.float32))
+    log("outputs of the last timed step: %d views x %d of %d pixels -> %s" % (len(bufs), n, h * w, path))
+
+
 def _protect_stdout():
     """Everything but the one JSON line goes to stderr: libraries (NCCL prints its version banner on stdout) must not
     pollute the line the driver parses.  Returns a file object bound to the original stdout."""
@@ -252,8 +272,11 @@ def _main(real_stdout):
     ap.add_argument("--workload", default="C2")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write depth / conf / dz of the last timed step to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
-    args.steps = max(1, args.steps)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(0, args.warmup)
     if args.impl == "reference":
         return reference_arm(args, real_stdout)
@@ -343,14 +366,14 @@ def _main(real_stdout):
 
     plan_wait, call_host = [0.0], [0.0]
 
-    def step_resident():
+    def step_resident(out=None):
         flush.zero_()
         t_w = time.perf_counter()
         pending.pop().result()
         plan_wait[0] += time.perf_counter() - t_w
         pending.append(planner.submit(gscene.plan_views, settings, refs))
         t_c = time.perf_counter()
-        _, st = gscene.reconstruct(settings, refs, download=False)
+        _, st = gscene.reconstruct(settings, refs, download=out is not None, out=out)
         call_host[0] += time.perf_counter() - t_c - 1e-3 * st.ms_total_device
         return st
 
@@ -376,13 +399,17 @@ def _main(real_stdout):
     barrier()
     stats = []
     plan_wait[0] = call_host[0] = 0.0
+    dump = args.dump_outputs and rank == 0
     with ClockSampler(local) as clk:
         t0 = time.perf_counter()
-        for _ in range(args.steps):
-            stats.append(step_resident())
+        for i in range(args.steps):
+            # the maps stay in HBM, except that the last step of a dumping run copies them to the pinned host buffers
+            stats.append(step_resident(out_bufs if dump and i == args.steps - 1 else None))
         barrier()
         elapsed = time.perf_counter() - t0
     clocks = clk.summary()
+    if dump:
+        dump_outputs(args.dump_outputs, out_bufs)
     filled_local = sum(int(s.n_filled) for s in stats)
     filled_total, _ = agg(filled_local)
     _, elapsed_max = agg(elapsed)

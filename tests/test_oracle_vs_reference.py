@@ -9,14 +9,12 @@ the restatement with strict IEEE evaluation; the reference differs from ITSELF b
 compiler flags (SURVEY.md §6: depth rel p99 3.2e-4, max 3.1e-3 at map level).  Integer results must be equal.
 """
 import os
-import subprocess
-import tempfile
 
 import numpy as np
 import pytest
 
 from oracle import oracle_py as O
-from tests.util import GOLD, ROOT, golden_ref, golden_scene, map_stats, patch_compare
+from tests.util import GOLD, golden_ref, golden_scene, map_stats, patch_compare, scene_sha256
 
 
 @pytest.fixture(scope="module")
@@ -106,22 +104,17 @@ def test_maps_vs_reference_cli(osc, name, views):
         assert np.percentile(np.abs(ref["dz_%d" % v] - r["dz"])[both], 99) < tol["dz"]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_harness")),
-                    reason="oracle/_ref not built (needs /root/reference)")
 def test_live_reference_patches_on_fresh_scene():
-    """Live run of the compiled reference on a scene that is NOT in the fixtures."""
+    """The compiled reference on a scene that the other fixtures do not use (rendered by the test, only its SHA-256 is
+    stored): its results for the first 3000 optimisations of the restatement's strict-order run of view 1."""
     from mve_b200 import synth
     s = synth.make_scene("T0", seed=77, features=200)
+    ref = golden_ref("T0_seed77")
+    assert scene_sha256(s) == str(ref["scene_sha256"])
     sc = O.OracleScene(s)
     st = O.default_settings(scale=0, nr_recon_neighbors=4)
-    r = sc.reconstruct(st, 1, trace_cap=3000)
-    with tempfile.TemporaryDirectory() as tmp:
-        synth.write_mve_scene(s, tmp)
-        fin, fout = os.path.join(tmp, "in.bin"), os.path.join(tmp, "out.bin")
-        r["trace_in"].tofile(fin)
-        subprocess.run([os.path.join(ROOT, "oracle", "_ref", "ref_harness"), "patches", tmp, "1", "0", "4", fin, fout],
-                       check=True, capture_output=True)
-        ref_out = np.fromfile(fout, dtype=O.PATCH_OUT)
-    c = patch_compare(r["trace_out"], ref_out)
+    assert sc.global_view_selection(st, 1) == ref["patch_gvs"].tolist()
+    got = sc.optimize_patches(st, 1, ref["patch_gvs"].tolist(), ref["patch_in"])
+    c = patch_compare(got, ref["patch_out"])
     assert c["ok_mismatch"] <= 3 and c["ids_mismatch"] <= 3
     assert np.percentile(c["rel"], 99) < 2e-5
